@@ -145,6 +145,18 @@ def build_workload(api, seed):
     return g, ids
 
 
+def dump_outputs(out_dir, api, ids, chi2):
+    """What a caller of the timed solve receives, as float64 .npy files in `out_dir`: the estimates of every pose (x y z qx qy
+    qz qw) and plane (a b c d), chi2 of the final estimate and the LM trace (lambda and accepted flag per trial step).  The
+    workload is generated from a fixed seed, so two builds of the project can be compared output for output (about 0.3 MB)."""
+    os.makedirs(out_dir, exist_ok=True)
+    tr = api.trace()
+    arrays = {"poses": api.get_poses(ids["pose_ids"]), "planes": api.get_planes(ids["plane_ids"]), "chi2": np.array([chi2]),
+              "lm_lambda": tr["lam"], "lm_accepted": tr["accepted"]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_reference(args, rank, world):
     """CPU arm: the oracle in its faithful mode (numeric Jacobians, ordering recomputed per solve)."""
     if rank != 0:
@@ -157,7 +169,7 @@ def run_reference(args, rank, world):
         api = OracleAPI()
         api.set_jacobian_mode(0)
         api.set_reuse_ordering(0)
-        gg.build_bulk(api, g)
+        ids = gg.build_bulk(api, g)
         gg.configure(api, g)
         t0 = time.perf_counter()
         it = api.batch_optimize()
@@ -165,6 +177,8 @@ def run_reference(args, rank, world):
         if step >= args.warmup:
             times.append(dt); iters.append(it)
         tm = api.timers()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, api, ids, api.chi2())
     total_t, total_it = sum(times), sum(iters)
     value = total_it / total_t
     # oracle/_ref (the unmodified reference sources compiled against the Eigen / CHOLMOD API shims) solves the same graph with
@@ -233,6 +247,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-batch64", action="store_true")
     ap.add_argument("--no-stress", action="store_true", help="skip the config-5 (HBM-bound) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the estimates, chi2 and LM trace of the last timed solve to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -287,6 +303,8 @@ def main():
     clocks = sampler.stop()
     ms_res = [a.elapsed_time(b) for a, b in ev]
     api.download()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, api, ids, stats_res[-1]["chi2_final"])
 
     # ---------------- end-to-end arm: host buffers in, host buffers out, through the C-ABI ----------------
     pose_host = torch.from_numpy(g.poses_init.copy()).pin_memory().numpy()

@@ -2,9 +2,9 @@
 Optimizer / Cholesky / numericalDiff, slam3d.h, isam_plane3d.{h,cpp}) compiled against the API shims of oracle/ref_shim
 (recipe: `make -C oracle ref`, needs the reference checkout; the built library travels to the GPU box).
 
-Test infrastructure only -- never imported by the product.  Tests that need it skip when the library is absent (a
-checkout without /root/reference that never ran `make ref`); the committed fixtures tests/golden/reference_build.json
-(generated from it by tools/make_ref_golden.py) carry its outputs in that case."""
+Test infrastructure only -- never imported by the product or the tests.  The fixture generators tools/make_ref_golden.py
+and tools/make_ref_build_golden.py run it to write tests/golden/reference_build.json and reference_build_*.npz, which
+carry its outputs to the tests; bench.py --impl reference also times it when the library has been built."""
 import ctypes as C
 import os
 import subprocess

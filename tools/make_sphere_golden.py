@@ -5,10 +5,13 @@ container; the committed JSON travels to the GPU box):
       (ISAM/isam/Loader.cpp:316-365: EDGE3 i j x y z roll pitch yaw + 21 sqrt-information entries, rotational block
       re-ordered to yaw, pitch, roll; prior sqrt-information 100*I on the first pose) together with the oracle's
       Gauss-Newton result on it (numeric Jacobians as upstream): chi2 before / after, iterations, every 8th pose.
+  tests/golden/sphere2500.txt.xz, tests/golden/sphere2500_groundtruth.txt.xz  -- ISAM/data/sphere2500.txt and
+      data/groundtruth/sphere2500_groundtruth.txt, byte for byte, xz-compressed.
 
 Regenerate with:  python tools/make_sphere_golden.py
 """
 import json
+import lzma
 import os
 import sys
 
@@ -24,9 +27,9 @@ DATA = "/root/reference/pop_planar_slam/Thirdparty/isam/data"
 
 
 def load_edge3(path):
-    """[(i, j, meas[x y z yaw pitch roll], sqrtinf packed upper-triangular 21)] in file order"""
+    """[(i, j, meas[x y z yaw pitch roll], sqrtinf packed upper-triangular 21)] in file order (.xz files are decompressed)"""
     edges = []
-    for line in open(path):
+    for line in (lzma.open(path, "rt") if path.endswith(".xz") else open(path)):
         tok = line.split()
         if not tok or tok[0] != "EDGE3":
             continue
@@ -71,3 +74,9 @@ if __name__ == "__main__":
     path = os.path.join(ROOT, "tests", "golden", "sphere400.json")
     json.dump(out, open(path, "w"))
     print("sphere400:", len(ids), "poses", len(edges), "edges; chi2", c0, "->", c1, "in", it, "iterations; wrote", path, os.path.getsize(path), "bytes")
+
+    for src in ("sphere2500.txt", "groundtruth/sphere2500_groundtruth.txt"):
+        path = os.path.join(ROOT, "tests", "golden", os.path.basename(src) + ".xz")
+        with lzma.open(path, "wb", preset=9 | lzma.PRESET_EXTREME) as f:
+            f.write(open(os.path.join(DATA, src), "rb").read())
+        print("wrote", path, os.path.getsize(path), "bytes")
